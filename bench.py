@@ -410,6 +410,27 @@ class KernelTimer:
         return agg
 
 
+DUMP_MAX_ELEMS = 1 << 21        # 8 MB of float32 per array: the six arrays of a dump stay under 64 MB
+DUMP_SEED = 20240917
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes every array as out_dir/<name>.npy in float32.  An array of more than DUMP_MAX_ELEMS elements is written as a
+    flat sample of DUMP_MAX_ELEMS elements at sorted positions drawn with a fixed seed from its size, so two runs of the
+    same config sample the same positions.  The inputs and weights of a run are fixed by its arguments, but the kernels
+    reduce with floating-point atomics and every step trains on the last one's update, so two runs agree to rounding
+    amplified over the steps, not bit for bit: compare dumps with a tolerance."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        v = t.detach()
+        if v.numel() > DUMP_MAX_ELEMS:
+            g = torch.Generator().manual_seed(DUMP_SEED)
+            idx = torch.randint(v.numel(), (DUMP_MAX_ELEMS,), generator=g).sort().values
+            v = v.reshape(-1)[idx.to(v.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), v.float().cpu().numpy())
+
+
 def bucket_checksum(params):
     """Integer checksum of the parameter bits (identical on every rank iff the parameters are)."""
     acc = torch.zeros(2, dtype=torch.int64, device=params[0].device)
@@ -461,11 +482,15 @@ def run_b200(args):
         [{"params": hp, "lr": TRAIN["lr"], "weight_decay": TRAIN["decay"]}], warmup=TRAIN["warmup"],
         t_total=TRAIN["t_total"], grad_clip=TRAIN["grad_clip"], bucket=bucket)
 
+    last = {}
+
     def compute():
         bucket.zero()
         feat.grad = None
         curr.grad = None
         logits = net.hot_path(feat, curr, None, sp)
+        if args.dump_outputs:
+            last["logits"] = logits             # in a captured step: the graph's buffer, rewritten by every replay
         loss, _, _ = seg_loss(logits, Y, pw, cw, TRAIN["dice_w"])         # train3d.py:731-756
         loss.backward()
         if world > 1 and not args.no_overlap:
@@ -525,6 +550,13 @@ def run_b200(args):
         dist.all_reduce(lo, op=dist.ReduceOp.MIN)
         dist.all_reduce(hi, op=dist.ReduceOp.MAX)
         checksum_agree = bool(torch.equal(lo, hi))
+    if args.dump_outputs and rank == 0:
+        # what the last timed step hands its caller: loss, logits, gradients of both feature tensors and of every
+        # hot-path parameter, and the parameters after the update
+        dump_outputs(args.dump_outputs, {
+            "loss": loss, "logits": last["logits"], "grad_feat": feat.grad, "grad_curr": curr.grad,
+            "param_grads": torch.cat([(torch.zeros_like(p) if p.grad is None else p.grad).reshape(-1) for p in hp]),
+            "params": torch.cat([p.detach().reshape(-1) for p in hp])})
 
     # ---- the same K steps again with a CUDA-event pair around every C-ABI call (per-kernel durations for the
     #      roofline; the extra event records cost host time, so this pass is not the headline number) ----
@@ -761,7 +793,15 @@ def main():
     ap.add_argument("--no-fused-attn", action="store_true", help="squeeze-out attention as separate GEMM + softmax kernels")
     ap.add_argument("--no-overlap", action="store_true", help="N>1: one all-reduce of the whole bucket after the step")
     ap.add_argument("--no-graph", action="store_true", help="enqueue every kernel from Python instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (loss, logits, feature and parameter "
+                         "gradients, updated parameters) as DIR/<name>.npy in float32; arrays of more than %d elements "
+                         "as a fixed seeded sample" % DUMP_MAX_ELEMS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the b200 step")
     wd = float(os.environ.get("SEGTRAN_BENCH_WATCHDOG_S", "0"))
     if wd == 0 and args.impl != "reference" and int(os.environ.get("WORLD_SIZE", "1")) > 1:
         wd = 900.0                                 # a multi-rank run takes ~1 min: a stalled collective must not hang the launcher

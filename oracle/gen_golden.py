@@ -239,6 +239,70 @@ def gen_poly(name="poly2d_tiny", seed=31):
     print(name, "out", tuple(y.shape), "max|out|", float(y.abs().max()))
 
 
+INIT_CASES = [([64, 64], 4, 16, 3, True), ([64, 64, 32], 4, 8, 2, False)]
+
+
+def gen_construction():
+    """What the construction tests compare against, recorded from the reference modules (digests where the test needs
+    exact equality, values where it needs numbers):
+      init_seed3.pt     encoders of INIT_CASES built with seed 3: state_dict order and digests, named_parameters order;
+      seg3d_init.pt     the Segtran3d shell of seg3d_tiny's args built with seed 3: every state_dict name, the backbone's
+                        tensor shapes, the CPU RNG state before (digest) and after (value) the backbone's construction,
+                        and the digests of every non-backbone tensor;
+      enc_train.pt      a fresh encoder config in train() mode (dropout 0): weights, inputs and output."""
+    from tests.helpers import state_digests, tensor_digest
+    ns = R.load()
+    cases = {}
+    for dims, M, A, pd, qkb in INIT_CASES:
+        cfg = R.encoder_config(ns.shared, dims=dims, num_modes=M, num_attractors=A, pos_dim=pd, qk_have_bias=qkb)
+        enc = R.build_encoder(cfg, seed=3)
+        cases[repr((dims, M, A, pd, qkb))] = dict(state_digests=state_digests(enc.state_dict()),
+                                                  param_names=[n for n, _ in enc.named_parameters()])
+    torch.save(dict(kind="init", seed=3, cases=cases), os.path.join(OUT, "init_seed3.pt"))
+    print("init_seed3", list(cases))
+
+    ns.shared.bb2feat_dims["i3d-tiny"] = [8, 16, 24, 32, 48]
+    args = Namespace(**torch.load(os.path.join(OUT, "seg3d_tiny.pt"), weights_only=False)["args"])
+    rng = {}
+    i3d = ns.seg3d.InceptionI3d
+
+    def recording_i3d(*a, **kw):
+        rng["before"] = torch.get_rng_state()
+        net = i3d(*a, **kw)
+        rng["after"] = torch.get_rng_state()
+        return net
+
+    ns.seg3d.InceptionI3d = recording_i3d
+    try:
+        torch.manual_seed(3)
+        with R.quiet():
+            ns.seg3d.CONFIG.update_config(args)
+            net = ns.seg3d.Segtran3d(ns.seg3d.CONFIG)
+    finally:
+        ns.seg3d.InceptionI3d = i3d
+    sd = net.state_dict()
+    torch.save(dict(kind="seg3d_init", seed=3, names=list(sd),
+                    backbone_shapes={k: tuple(v.shape) for k, v in sd.items() if k.startswith("backbone.")},
+                    rng_before_backbone=tensor_digest(rng["before"]), rng_after_backbone=rng["after"],
+                    state_digests=state_digests({k: v for k, v in sd.items() if not k.startswith("backbone.")})),
+               os.path.join(OUT, "seg3d_init.pt"))
+    print("seg3d_init", len(sd), "tensors")
+
+    dims = [32, 32, 16]
+    cfg = R.encoder_config(ns.shared, dims=dims, num_modes=2, num_attractors=5, pos_dim=2, qk_have_bias=True)
+    enc = R.build_encoder(cfg, seed=11).train()
+    torch.manual_seed(12)
+    x = torch.randn(3, 20, 32)
+    pos = O.voxels_pos_for_grid((4, 5), (8, 8), 3)
+    mask = torch.ones(3, 20, 1, dtype=torch.bool)
+    with R.quiet():
+        y = enc(x, pos, mask, torch.Size((4, 5)))
+    torch.save(dict(kind="enc_train", dims=dims, num_modes=2, grid=[4, 5], x=x, voxels_pos=pos, vmask=mask,
+                    state_dict=dict(enc.state_dict()), out=y.detach()),
+               os.path.join(OUT, "enc_train.pt"))
+    print("enc_train out", tuple(y.shape))
+
+
 def gen_infer():
     """Sliding-window inference fixtures produced by the reference's own test_util3d.test_single_case (un-padded volumes:
     the reference's padding branch hands F.pad the pads in the wrong dimension order, test_util3d.py:119-120, and cannot run)."""
@@ -293,6 +357,9 @@ def main():
         return
     if len(sys.argv) > 1 and sys.argv[1] == "poly":
         gen_poly()
+        return
+    if len(sys.argv) > 1 and sys.argv[1] == "construction":
+        gen_construction()
         return
     if len(sys.argv) > 1 and sys.argv[1] == "variants":
         gen_encoder("enc2d_nosqueeze", [64, 64], 4, 8, 2, True, (6, 7), 2, seed=21, squeeze=False)

@@ -1,4 +1,5 @@
 """Shared test helpers (tolerances, fixture loading, oracle drivers)."""
+import hashlib
 import os
 
 import torch
@@ -17,6 +18,20 @@ def rel_err(a, b):
     a = a.detach().double().cpu()
     b = b.detach().double().cpu()
     return float((a - b).abs().max() / b.abs().max().clamp_min(1e-30))
+
+
+def tensor_digest(t):
+    """SHA-256 of a tensor's dtype, shape and bytes: two tensors have the same digest iff they are bit-identical, so a
+    fixture can pin exact values without storing them."""
+    t = t.detach().cpu().contiguous()
+    h = hashlib.sha256(("%s %s" % (t.dtype, tuple(t.shape))).encode())
+    h.update(t.reshape(-1).view(torch.uint8).numpy().tobytes())
+    return h.hexdigest()
+
+
+def state_digests(sd):
+    """name -> tensor_digest, in state_dict order."""
+    return {k: tensor_digest(v) for k, v in sd.items()}
 
 
 def rms_rel(a, b):

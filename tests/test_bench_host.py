@@ -39,6 +39,23 @@ def test_weak_and_strong_batch_split():
         bench.local_batch(c, Namespace(scaling="strong"), 8)                # 4 samples do not split over 8 GPUs
 
 
+def test_dump_outputs_writes_float32_and_samples_large_arrays_reproducibly(tmp_path):
+    import numpy as np
+    import torch
+    n = bench.DUMP_MAX_ELEMS + 1000
+    big = torch.arange(n, dtype=torch.float64)
+    small = torch.randn(3, 4, dtype=torch.bfloat16)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"big": big, "small": small, "loss": torch.tensor(1.5)})
+    a = {k: np.load(str(tmp_path / "a" / (k + ".npy"))) for k in ("big", "small", "loss")}
+    assert all(v.dtype == np.float32 for v in a.values())
+    assert np.array_equal(a["small"], small.float().numpy()) and a["loss"].shape == () and float(a["loss"]) == 1.5
+    # a sorted sample of positions drawn with a fixed seed: the same positions in every run, all in range
+    assert a["big"].shape == (bench.DUMP_MAX_ELEMS,) and np.all(np.diff(a["big"]) >= 0) and a["big"][-1] < n
+    assert len(np.unique(a["big"])) > bench.DUMP_MAX_ELEMS // 2
+    assert np.array_equal(a["big"], np.load(str(tmp_path / "b" / "big.npy")))
+
+
 def test_reference_arm_is_silent_on_other_ranks():
     """Under torchrun the driver starts `bench.py --impl reference` on every rank: only rank 0 works and prints."""
     env = dict(os.environ, RANK="1", LOCAL_RANK="1", WORLD_SIZE="2", MASTER_ADDR="127.0.0.1", MASTER_PORT="29999")
